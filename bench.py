@@ -14,6 +14,11 @@ One "step" = one full pass of the workload over one batch:
   vqgan     configs[4]: f4 VQGAN encode -> indices -> decode_indices round trip, bs=256/GPU, 256x256 images
 Prints ONE JSON line (rank 0).
 
+  --dump-outputs DIR  rank 0 writes what the timed (HBM-resident) path returned in its last timed step as float32 .npy
+                      files: tokens.npy for the sample workloads, images_sample.npy + images_sample_index.npy (a fixed,
+                      seeded sample of the decoded images and its flat indices) for vqgan.  Inputs and seeds depend only
+                      on the arguments, so two builds run with the same arguments can be compared output for output.
+
   value     images/s with the inputs already resident in HBM
   e2e       images/s through the public API with HOST (pinned) inputs: H2D of the step's inputs and D2H of its result
             inside the timed region, every step
@@ -31,6 +36,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -56,6 +62,7 @@ WORKLOADS = {
 # kept as module constants for tools/ that import bench
 LATENT, SAMPLE_STEPS, RENOISE, BATCH = 32, 8, 7, 64
 METRIC, WORKLOAD = WORKLOADS["sample"]["metric"], WORKLOADS["sample"]["desc"]
+DUMP_MAX_ELEMS = 1 << 22    # --dump-outputs: larger outputs are sampled (4 Mi float32 values + float64 indices = 48 MB)
 
 
 def log(msg):
@@ -146,6 +153,17 @@ def ncu_traffic():
         except (OSError, KeyError, ValueError, ZeroDivisionError):
             continue
     return None, None
+
+
+def dump_arrays(name, out):
+    """--dump-outputs: one output tensor as float32 arrays, whole up to DUMP_MAX_ELEMS elements, else a fixed seeded sample
+    of its flattened elements plus their flat indices (float64, exact)."""
+    out = out.detach()
+    if out.numel() <= DUMP_MAX_ELEMS:
+        return {name: out.float().cpu().numpy()}
+    idx = torch.randint(out.numel(), (DUMP_MAX_ELEMS,), generator=torch.Generator().manual_seed(0)).sort().values
+    return {f"{name}_sample": out.reshape(-1)[idx.to(out.device)].float().cpu().numpy(),
+            f"{name}_sample_index": idx.double().numpy()}
 
 
 def build_model(device):
@@ -333,7 +351,11 @@ def main():
     ap.add_argument("--ref-batch", type=int, default=1)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cuda-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after timing, write the last timed step's outputs to DIR as float32 .npy files "
+                    "(the tokens; for vqgan a fixed, seeded sample of the images)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -372,6 +394,7 @@ def main():
 
         def step_resident():
             return vq.decode_indices(vq.encode(img_d)[2])
+        dump_name = "images"
 
         def step_e2e():
             x = img_h.to(dev, non_blocking=True)
@@ -391,6 +414,7 @@ def main():
 
         def step_resident():
             return U.sample(model, cond_d, shape, uncond_d, **kw)
+        dump_name = "tokens"
 
         host_tokens = torch.empty(shape, dtype=torch.int64).pin_memory()
 
@@ -423,15 +447,16 @@ def main():
         torch.cuda.synchronize()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        for _ in range(steps):
+        for _ in range(steps - 1):
             fn()
+        last = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
             dist.barrier()
-        return float(ms)
+        return float(ms), last
 
     log(f"rank {rank}: weights packed; warm-up x{max(args.warmup, 3)}")
     for _ in range(max(args.warmup, 3)):
@@ -440,12 +465,14 @@ def main():
     log(f"timing {args.steps} steps (HBM-resident inputs)")
     launches0 = L.pb200_launch_count()
     with ClockSampler(local_rank) as clk:
-        ms = timed(step_resident, args.steps)
+        ms, last = timed(step_resident, args.steps)
     launches = L.pb200_launch_count() - launches0
+    dumped = dump_arrays(dump_name, last) if args.dump_outputs and rank == 0 else {}
+    del last
     log(f"  {ms / args.steps:.1f} ms/step; timing {args.steps} steps end to end (host inputs)")
     for _ in range(2):
         step_e2e()
-    ms_e2e = timed(step_e2e, args.steps)
+    ms_e2e, _ = timed(step_e2e, args.steps)
     log(f"  {ms_e2e / args.steps:.1f} ms/step; profiled step")
     value = world * B * args.steps / (ms / 1e3)
     e2e = world * B * args.steps / (ms_e2e / 1e3)
@@ -460,7 +487,7 @@ def main():
                 return U.sample(model, cond_d, shape, uncond_d, decode=vq, **kw)
             for _ in range(2):
                 step_dec()
-            ms_dec = timed(step_dec, args.steps)
+            ms_dec, _ = timed(step_dec, args.steps)
             extra["with_decode"] = {"value": B * args.steps / (ms_dec / 1e3), "unit": "images/s", "ms_per_step": ms_dec / args.steps,
                                     "what": "sample(..., decode=vqmodel): tokens -> f4 VQGAN decode_indices -> clamp(0,1) -> uint8 NHWC, on-stream"}
         except Exception as e:  # noqa: BLE001
@@ -529,6 +556,11 @@ def main():
         except Exception as e:  # noqa: BLE001
             out["cpu_baseline"] = {"value": None, "unit": "images/s", "cores": host_threads(), "kind": "reference",
                                    "sample": f"not measured: {type(e).__name__} (300 s limit)"}
+    if dumped:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for k, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{k}.npy"), a)
+        log(f"outputs of the last timed step: {', '.join(f'{k}{list(a.shape)}' for k, a in dumped.items())} -> {args.dump_outputs}")
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -1,15 +1,15 @@
 #!/usr/bin/env python
 """Generate the committed golden fixtures by running the REAL reference on CPU.
 
-Run in the dev container only (needs /root/reference):
-    python tests/golden/make_golden.py
+Needs a checkout of the original dome272/Paella, named by PAELLA_REFERENCE:
+    PAELLA_REFERENCE=<checkout> python tests/golden/make_golden.py
 It imports ref/src/modules.py, ref/utils/modules.py, ref/utils/alter_attention.py,
 ref/src/vqgan.py and ref/src/utils.py UNMODIFIED.  ``torchtools`` (third-party,
 absent) is stubbed only so those files import; the stub's quantiser is our
 restatement (oracle/vqgan_oracle.py) and is NOT what these fixtures pin — the
 fixtures record the conv stacks' pre-quantisation latents and decoder outputs.
 
-Outputs (small, committed):  tests/golden/paella_tiny.npz, vqgan_tiny.npz, sample_tiny.npz
+Outputs (small, committed):  tests/golden/paella_tiny.npz, vqgan_tiny.npz, sample_tiny.npz, reference_default.npz
 """
 import importlib.util
 import os
@@ -22,11 +22,11 @@ from torch import nn
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-REF = os.environ.get("PAELLA_REFERENCE", "/root/reference")
+REF = os.environ.get("PAELLA_REFERENCE", "")
 sys.path.insert(0, ROOT)
 
 from oracle import vqgan_oracle as vo          # noqa: E402
-from paella_b200.synth import rerandomize_     # noqa: E402
+from paella_b200.synth import rerandomize_, synthetic_conditioning     # noqa: E402
 
 TINY = dict(c_in=16, c_out=16, num_labels=64, c_r=64, patch_size=2, c_cond=32, c_hidden=[32, 64, 64],
             nhead=[-1, 4, 4], blocks=[1, 2, 1], level_config=["CT", "CTA", "CTA"], clip_embd=24,
@@ -64,6 +64,8 @@ def load_by_path(name, path):
 
 
 def load_reference():
+    if not os.path.isdir(os.path.join(REF, "src")):
+        raise SystemExit("set PAELLA_REFERENCE to a checkout of dome272/Paella")
     install_torchtools_stub()
     ref_modules = load_by_path("ref_src_modules", os.path.join(REF, "src", "modules.py"))
     ref_nb_modules = load_by_path("ref_utils_modules", os.path.join(REF, "utils", "modules.py"))
@@ -82,6 +84,49 @@ def load_reference():
 
 def sd_to_np(sd, prefix):
     return {prefix + k: v.detach().cpu().numpy() for k, v in sd.items()}
+
+
+def fingerprint(tensors, prefix):
+    """Names plus float64 sum and sum of squares of every tensor: pins seeded data too large to store."""
+    ts = [v.detach().double() for v in tensors.values()]
+    return {prefix + "keys": np.array(list(tensors)), prefix + "sum": np.array([float(t.sum()) for t in ts]),
+            prefix + "sumsq": np.array([float(t.pow(2).sum()) for t in ts])}
+
+
+N_LOGIT_SAMPLES = 8192
+
+
+def make_reference_default(ref_modules, ref_vqgan):
+    """reference_default.npz: the reference-default denoiser (1.008 B) and f4 VQGAN, weights re-randomised from seeds.
+    Weights and the seeded float inputs are recorded as fingerprints, the 8.4 M denoiser logits as a seeded sample plus
+    their per-channel and per-position means; the token inputs and the codec outputs are stored whole."""
+    torch.manual_seed(0)
+    m = ref_modules.Paella(byt5_embd=2560).eval()
+    rerandomize_(m.state_dict(), seed=0)
+    cond, _ = synthetic_conditioning(1, 16, with_clip_image=True)
+    x = torch.randint(0, 8192, (1, 32, 32), generator=torch.Generator().manual_seed(1))
+    r = torch.tensor([0.6])
+    logits = m(x, r, cond["byt5"], clip=cond["clip"], clip_image=cond["clip_image"])
+    flat = logits.reshape(-1).numpy()
+    idx = np.sort(np.random.default_rng(0).choice(flat.size, N_LOGIT_SAMPLES, replace=False)).astype(np.int32)
+    out = {"x": x.numpy().astype(np.int16), "r": r.numpy(), "logits_shape": np.array(logits.shape),
+           "logits_std": np.array(float(logits.std())), "logits_idx": idx, "logits_sample": flat[idx],
+           "logits_channel_mean": logits.mean((0, 2, 3)).numpy(), "logits_position_mean": logits.mean(1).reshape(-1).numpy()}
+    out.update(fingerprint(cond, "cond_"))
+    out.update(fingerprint(m.state_dict(), "denoiser_sd_"))
+    del m, logits
+
+    torch.manual_seed(0)
+    vq = ref_vqgan.VQModel().eval()
+    rerandomize_(vq.state_dict(), seed=4)
+    img = torch.rand(1, 3, 64, 64, generator=torch.Generator().manual_seed(7))
+    idx_v = torch.randint(0, 8192, (1, 16, 16), generator=torch.Generator().manual_seed(8))
+    out.update({"vq_latents": vq.down_blocks(vq.in_block(img)).numpy(), "vq_idx": idx_v.numpy().astype(np.int16),
+                "vq_dec_indices": vq.decode_indices(idx_v).numpy()})
+    out.update(fingerprint({"img": img}, "vq_img_"))
+    out.update(fingerprint(vq.state_dict(), "vqgan_sd_"))
+    np.savez_compressed(os.path.join(HERE, "reference_default.npz"), **out)
+    print("reference_default.npz:", {k: v.shape for k, v in out.items()})
 
 
 def main():
@@ -185,6 +230,8 @@ def main():
     vo_.update(sd_to_np(vsd, "sd:"))
     np.savez_compressed(os.path.join(HERE, "vqgan_tiny.npz"), **vo_)
     print("vqgan_tiny.npz:", {k: v.shape for k, v in vo_.items() if not k.startswith("sd:")})
+
+    make_reference_default(ref_modules, ref_vqgan)
 
 
 if __name__ == "__main__":

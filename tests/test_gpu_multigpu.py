@@ -1,5 +1,5 @@
 """Multi-GPU data-plane tests (SURVEY.md §8e; VERDICT r1 "missing" #7, ADVICE r1 high/medium): world_size-2 NCCL, one
-process per GPU, spawned from the test.  Skipped on boxes with one GPU (run with `gpurun --gpus 2`).
+process per GPU, spawned from the test.  Skipped on machines with fewer than two GPUs.
 
   * per-shard parity: rank r's shard of a sharded sample() == a SINGLE-GPU run of that shard's inputs with that shard's seed
     (parallel.shard_range / rank_seed / gather_tokens used for real)
@@ -82,7 +82,7 @@ def _worker(rank, world, port, ret):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs (gpurun --gpus 2)")
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs 2 GPUs")
 def test_two_gpu_per_shard_parity_and_broadcast_weights():
     import torch.multiprocessing as mp
     from helpers import load_golden
