@@ -275,6 +275,12 @@ int pb200_paella_logits(pb200_paella* m, const float* features, int batch, int h
 int pb200_paella_sample_tokens(pb200_paella* m, const float* features, int batch, int hw, int cfg_on, double cfg,
                                double temperature, uint64_t seed, uint64_t offset, int64_t* tokens_out,
                                void* workspace, int64_t workspace_bytes, void* stream);
+/* Masked (inpainting) form of pb200_paella_sample_tokens: tokens_inout int64 [B*HW] holds the known tokens on entry;
+ * rows with mask[row] != 0 (uint8 [B*HW], 1 = regenerate) receive exactly the token pb200_paella_sample_tokens would
+ * write there for the same (seed, offset); rows with mask 0 are not written.  Work scales with the rows to regenerate. */
+int pb200_paella_sample_tokens_masked(pb200_paella* m, const float* features, int batch, int hw, int cfg_on, double cfg,
+                                      double temperature, uint64_t seed, uint64_t offset, const uint8_t* mask,
+                                      int64_t* tokens_inout, void* workspace, int64_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * VQGAN (ref/src/vqgan.py:45-107).
@@ -329,6 +335,12 @@ int pb200_vq_mlp_fused(const void* a16, int64_t rows, int c, const void* w1_f16,
 enum { PB200_IMG_F32_NCHW = 0, PB200_IMG_F32_NCHW_CLAMP01 = 1, PB200_IMG_U8_NHWC = 2 };
 int pb200_vqgan_decode_ex(pb200_vqgan* m, const int64_t* indices, const float* latents_nchw, int batch, int h, int w,
                           void* img, int img_mode, void* workspace, int64_t workspace_bytes, void* stream);
+/* decode_ex of indices int64 [B,h,w] composited into an original image: where pixel_mask (uint8 [B,4h,4w]) is 0 the
+ * output pixel is orig_img (fp32 NCHW [B,3,4h,4w]) put through the same img_mode conversion, elsewhere the decoded
+ * pixel.  The compositing happens in the decoder's last kernel (inpainting with the untouched pixels pasted back). */
+int pb200_vqgan_decode_composite(pb200_vqgan* m, const int64_t* indices, int batch, int h, int w, const float* orig_img,
+                                 const uint8_t* pixel_mask, void* img, int img_mode, void* workspace,
+                                 int64_t workspace_bytes, void* stream);
 
 /* Re-read the host-mirrored scalars (the six ResBlock gammas, kernel arguments) from the bound weight blob.  Needed when
  * the blob was filled by anything other than pb200_vqgan_load_param on this handle (NCCL broadcast, a packed file,

@@ -98,6 +98,8 @@ SIGNATURES = {
     "pb200_paella_logits": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p, c_void_p, c_int64, c_void_p]),
     "pb200_paella_sample_tokens": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_double, c_uint64,
                                            c_uint64, c_void_p, c_void_p, c_int64, c_void_p]),
+    "pb200_paella_sample_tokens_masked": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_double, c_double, c_uint64,
+                                                  c_uint64, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "pb200_vqgan_create": (c_int, [POINTER(VqganConfig), POINTER(c_void_p)]),
     "pb200_vqgan_destroy": (None, [c_void_p]),
     "pb200_vqgan_weight_bytes": (c_int64, [c_void_p]),
@@ -113,6 +115,8 @@ SIGNATURES = {
                                    c_void_p]),
     "pb200_vqgan_decode_ex": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_void_p, c_int64,
                                       c_void_p]),
+    "pb200_vqgan_decode_composite": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int,
+                                             c_void_p, c_int64, c_void_p]),
     "pb200_vqgan_sync_params": (c_int, [c_void_p, c_void_p]),
     "pb200_vq_mlp_fused": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_void_p]),
     "pb200_vqgan_resblock_workspace_bytes": (c_int64, [c_int, c_int, c_int, c_int]),

@@ -549,7 +549,9 @@ int64_t pb200_paella_workspace_bytes(const pb200_paella* m, int batch_total, int
     // logits / sampling scratch: fp16 features for B*H*W rows
     // fp16 features of the sampler; the shared-Philox kernel reads whole 4*rs-row blocks (rs <= 1184*256/num_labels + 1)
     const int64_t pad_rows = 4 * ((int64_t)1184 * 256 / m->cfg.num_labels + 2);
-    const int64_t samp = (((int64_t)batch_total * h * w + pad_rows) * m->cfg.c_out * 2 + 255) / 256 * 256;
+    const int64_t samp_rows = (int64_t)batch_total * h * w + pad_rows;
+    // + the needed-slot list of the masked sampler (pb200_paella_sample_tokens_masked)
+    const int64_t samp = (samp_rows * m->cfg.c_out * 2 + 255) / 256 * 256 + 256 + (samp_rows + 255) / 256 * 256;
     int64_t need = a.off > b.off ? a.off : b.off;
     need = need > samp ? need : samp;
     return need + 256;
@@ -872,6 +874,29 @@ int pb200_paella_sample_tokens(pb200_paella* m, const float* features, int batch
         PB_TRY(launch_cast_f16(features, rows * c.c_out, a16, st));
     return launch_fused_sampler(a16, rows, c.c_out, m->w<__half>(m->out_w), c.num_labels, 1.0f / (float)temperature, seed,
                                 offset, tokens_out, st);
+}
+
+int pb200_paella_sample_tokens_masked(pb200_paella* m, const float* features, int batch, int hw, int cfg_on, double cfg,
+                                      double temperature, uint64_t seed, uint64_t offset, const uint8_t* mask,
+                                      int64_t* tokens_inout, void* workspace, int64_t workspace_bytes, void* stream) {
+    PB_CHECK(m->blob != nullptr, "sample_tokens_masked: weights not bound");
+    PB_CHECK(mask != nullptr, "sample_tokens_masked: mask is required");
+    PB_CHECK(((uintptr_t)workspace & 255) == 0, "workspace must be 256-byte aligned");
+    const pb200_paella_config& c = m->cfg;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t rows = (int64_t)batch * hw;
+    const int64_t a16_bytes = (fused_sampler_rows_padded(rows, c.num_labels) * c.c_out * 2 + 255) / 256 * 256;
+    PB_CHECK(a16_bytes + fused_sampler_mask_scratch_bytes(rows, c.num_labels) <= workspace_bytes,
+             "sample_tokens_masked: workspace too small (use pb200_paella_workspace_bytes)");
+    PB_CHECK(temperature > 0, "sample_tokens_masked: temperature must be positive");
+    __half* a16 = reinterpret_cast<__half*>(workspace);
+    // the CFG mix / fp16 cast stays dense: it is one pass over c_out-wide rows, the sampler is the 8192-wide part
+    if (cfg_on)
+        PB_TRY(launch_mix_cast_f16(features, features + rows * c.c_out, (float)cfg, (float)(1.0 - cfg), rows * c.c_out, a16, st));
+    else
+        PB_TRY(launch_cast_f16(features, rows * c.c_out, a16, st));
+    return launch_fused_sampler_masked(a16, rows, c.c_out, m->w<__half>(m->out_w), c.num_labels, 1.0f / (float)temperature, seed,
+                                       offset, mask, reinterpret_cast<uint8_t*>(workspace) + a16_bytes, tokens_inout, st);
 }
 
 }  // extern "C"

@@ -30,9 +30,15 @@ constexpr int SMP_A_BYTES = 128 * 64 * 2;     // one k-block of the A tile
 constexpr int SMP_W_BYTES = SMP_BN * 64 * 2;
 constexpr int SMP_SMEM = SMP_MAX_KB * SMP_A_BYTES + SMP_STAGES * SMP_W_BYTES + 1024 + 256 + (SMP_EPI_WARPS / 4) * 128 * 8;
 
+// MASKED: only rows with mask[row] != 0 are written; a CTA whose 128 rows are all kept exits before its first TMA.
+template <bool MASKED>
 __global__ void __launch_bounds__(SMP_THREADS, 1)
 fused_sampler_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w, int R, int NL,
-                     int Kc, float inv_t, TorchPhilox rng, int64_t* __restrict__ out) {
+                     int Kc, float inv_t, TorchPhilox rng, const uint8_t* __restrict__ mask, int64_t* __restrict__ out) {
+    if constexpr (MASKED) {
+        const int r = blockIdx.x * 128 + (int)threadIdx.x;
+        if (!__syncthreads_or(threadIdx.x < 128 && r < R && mask[r] != 0)) return;
+    }
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -155,7 +161,7 @@ fused_sampler_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
         constexpr int NS = SMP_EPI_WARPS / 4;
         if (half > 0) { best_v[(half - 1) * 128 + row_in_tile] = bv; best_i[(half - 1) * 128 + row_in_tile] = bidx; }
         asm volatile("bar.sync 1, %0;" ::"n"(32 * SMP_EPI_WARPS) : "memory");
-        if (half == 0 && row_ok) {
+        if (half == 0 && row_ok && (!MASKED || mask[row] != 0)) {
 #pragma unroll
             for (int s = 0; s < NS - 1; ++s) {
                 const float ov = best_v[s * 128 + row_in_tile];
@@ -178,6 +184,12 @@ fused_sampler_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_cons
 // tile ordered (jj, g) -> row 4rs*i + rs*g + jj0 + jj (a 4-D TMA box, g innermost).  A thread then owns one label of
 // each 128-label chunk (TMEM lane) and 20 token columns = 5 Philox calls, keeps a running arg-max per column over the
 // 64 chunks in registers, and the 128 lanes are reduced once at the end.  ~2.9x fewer instructions per logit.
+//
+// SPARSE (masked sampling): the unit of work is a slot (blk, jj) = the 4 rows sharing one Philox call per label.  Task t
+// takes slots [20t, 20t+20) of the list masked_slot_list_kernel built (a slot is listed when any of its rows is masked)
+// and loads each with a {64, 4, 1, 1} box of the same 4-D view into the shared-memory rows 4i..4i+3 -- the rows, and
+// the 128B-swizzle phase (address bits 7-9), the dense box would give slot jj0 + i.  MMA, Philox and arg-max are the
+// dense ones per column, so a masked row gets exactly the dense draw; only masked rows are written.
 constexpr int SH_JJ = 20;                      // jj slots per task
 constexpr int SH_N = 4 * SH_JJ;                // token columns per MMA tile (UMMA N = 80)
 constexpr int SH_EPI_WARPS = 16;
@@ -207,9 +219,16 @@ __device__ __forceinline__ void tmem_ld_x4(uint32_t taddr, float* v) {
     for (int i = 0; i < 4; ++i) v[i] = __uint_as_float(r[i]);
 }
 
+template <bool SPARSE>
 __global__ void __launch_bounds__(SH_THREADS, 1)
 fused_sampler_shared_kernel(const __grid_constant__ CUtensorMap tm_f, const __grid_constant__ CUtensorMap tm_w, int R, int NL,
-                            int Kc, int rs, int tasks_per_block, float inv_t, TorchPhilox rng, int64_t* __restrict__ out) {
+                            int Kc, int rs, int tasks_per_block, float inv_t, TorchPhilox rng, const int* __restrict__ slots,
+                            const int* __restrict__ n_slots, const uint8_t* __restrict__ mask, int64_t* __restrict__ out) {
+    int ns = SH_JJ;                                                    // SPARSE: slots of this task
+    if constexpr (SPARSE) {
+        ns = min(SH_JJ, *n_slots - (int)blockIdx.x * SH_JJ);
+        if (ns <= 0) return;                                           // dense task count launched; the list is shorter
+    }
     extern __shared__ uint8_t smem_raw[];
     const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
     uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
@@ -254,9 +273,25 @@ fused_sampler_shared_kernel(const __grid_constant__ CUtensorMap tm_f, const __gr
     const uint32_t tmem_base = *reinterpret_cast<uint32_t*>(smem_gen + (tmem_slot - smem_base));
 
     if (warp == 0) {
+        if constexpr (SPARSE) {
+            // one slot per lane; the coordinates reach the TMA issue through a shuffle, which keeps them warp-uniform
+            const int nsw = __shfl_sync(0xffffffffu, ns, 0);
+            const int s = lane < nsw ? slots[blockIdx.x * SH_JJ + lane] : 0;
+            const int sb = s / rs, sj = s - sb * rs;
+            if (ptx::elect_one()) ptx::mbar_arrive_expect_tx(f_bar, n_kb * nsw * 4 * 128);
+            __syncwarp();
+            for (int kb = 0; kb < n_kb; ++kb)
+                for (int i = 0; i < nsw; ++i) {
+                    const int bi_ = __shfl_sync(0xffffffffu, sb, i), ji_ = __shfl_sync(0xffffffffu, sj, i);
+                    if (ptx::elect_one()) ptx::tma_load_4d(&tm_f, f_bar, f_base + kb * SH_F_BYTES + i * 4 * 128, kb * 64, 0, ji_, bi_);
+                    __syncwarp();
+                }
+        }
         if (ptx::elect_one()) {
-            ptx::mbar_arrive_expect_tx(f_bar, n_kb * SH_F_BYTES);
-            for (int kb = 0; kb < n_kb; ++kb) ptx::tma_load_4d(&tm_f, f_bar, f_base + kb * SH_F_BYTES, kb * 64, 0, jj0, blk);
+            if constexpr (!SPARSE) {
+                ptx::mbar_arrive_expect_tx(f_bar, n_kb * SH_F_BYTES);
+                for (int kb = 0; kb < n_kb; ++kb) ptx::tma_load_4d(&tm_f, f_bar, f_base + kb * SH_F_BYTES, kb * 64, 0, jj0, blk);
+            }
             int stage = 0;
             uint32_t phase = 0;
             for (int ch = 0; ch < n_chunks; ++ch)
@@ -300,6 +335,16 @@ fused_sampler_shared_kernel(const __grid_constant__ CUtensorMap tm_f, const __gr
         int bi[SH_JJ];
 #pragma unroll
         for (int i = 0; i < SH_JJ; ++i) { bv[i] = -INFINITY; bi[i] = 0x7fffffff; }
+        int sp_blk[SH_JJ / 4], sp_jj[SH_JJ / 4];                    // SPARSE: the (blk, jj) of this thread's 5 slots
+        if constexpr (SPARSE) {
+#pragma unroll
+            for (int c4 = 0; c4 < SH_JJ / 4; ++c4) {
+                const int i = sub * (SH_JJ / 4) + c4;
+                const int s = i < ns ? slots[blockIdx.x * SH_JJ + i] : 0;
+                sp_blk[c4] = s / rs;
+                sp_jj[c4] = s - sp_blk[c4] * rs;
+            }
+        }
         for (int ch = 0; ch < n_chunks; ++ch) {
             const int as = ch & 1;
             ptx::mbar_wait(tfull_bar(as), (ch >> 1) & 1);
@@ -315,8 +360,9 @@ fused_sampler_shared_kernel(const __grid_constant__ CUtensorMap tm_f, const __gr
             if (label < NL) {
 #pragma unroll
                 for (int c4 = 0; c4 < SH_JJ / 4; ++c4) {
-                    const int jj = jj0 + sub * (SH_JJ / 4) + c4;
-                    const uint4 r4 = torch_philox_call(rng, (uint64_t)jj * (uint64_t)NL + (uint64_t)label, (uint64_t)blk);
+                    const int jj = SPARSE ? sp_jj[c4] : jj0 + sub * (SH_JJ / 4) + c4;
+                    const int pb = SPARSE ? sp_blk[c4] : blk;
+                    const uint4 r4 = torch_philox_call(rng, (uint64_t)jj * (uint64_t)NL + (uint64_t)label, (uint64_t)pb);
                     const uint32_t bits[4] = {r4.x, r4.y, r4.z, r4.w};
 #pragma unroll
                     for (int g = 0; g < 4; ++g) {
@@ -352,14 +398,52 @@ fused_sampler_shared_kernel(const __grid_constant__ CUtensorMap tm_f, const __gr
                 const int oi = red_i[qq * SH_N + t];
                 if (ov > best || (ov == best && oi < besti)) { best = ov; besti = oi; }
             }
-            const int jj = jj0 + t / 4, g = t & 3;
-            const int64_t row = (int64_t)blk * 4 * rs + (int64_t)g * rs + jj;
-            if (jj < rs && row < R) out[row] = besti;
+            if constexpr (SPARSE) {
+                if (t / 4 < ns) {
+                    const int s = slots[blockIdx.x * SH_JJ + t / 4];
+                    const int sb = s / rs;
+                    const int64_t row = (int64_t)sb * 4 * rs + (int64_t)(t & 3) * rs + (s - sb * rs);
+                    if (row < R && mask[row] != 0) out[row] = besti;
+                }
+            } else {
+                const int jj = jj0 + t / 4, g = t & 3;
+                const int64_t row = (int64_t)blk * 4 * rs + (int64_t)g * rs + jj;
+                if (jj < rs && row < R) out[row] = besti;
+            }
         }
     }
     ptx::tc_fence_before();
     __syncthreads();
     if (warp == 1) ptx::tmem_dealloc(tmem_base, 256);
+}
+
+// Masked sampling: lists the slots (blk, jj) with at least one masked row, in slot order within a CTA (the order across
+// CTAs follows the atomics and does not affect the draws).  *count must be zero on entry.
+__global__ void __launch_bounds__(256) masked_slot_list_kernel(const uint8_t* __restrict__ mask, int64_t R, int rs, int n_slots,
+                                                                int* __restrict__ slots, int* __restrict__ count) {
+    __shared__ int warp_n[8];
+    __shared__ int base;
+    const int s = blockIdx.x * 256 + threadIdx.x;
+    bool need = false;
+    if (s < n_slots) {
+        const int blk = s / rs, jj = s - blk * rs;
+#pragma unroll
+        for (int g = 0; g < 4; ++g) {
+            const int64_t row = (int64_t)blk * 4 * rs + (int64_t)g * rs + jj;
+            need |= row < R && mask[row] != 0;
+        }
+    }
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const uint32_t bal = __ballot_sync(0xffffffffu, need);
+    if (lane == 0) warp_n[warp] = __popc(bal);
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int tot = 0;
+        for (int w = 0; w < 8; ++w) { const int n = warp_n[w]; warp_n[w] = tot; tot += n; }
+        base = tot ? atomicAdd(count, tot) : 0;
+    }
+    __syncthreads();
+    if (need) slots[base + warp_n[warp] + __popc(bal & ((1u << lane) - 1u))] = s;
 }
 
 int64_t fused_sampler_rows_padded(int64_t R, int NL) {
@@ -369,8 +453,14 @@ int64_t fused_sampler_rows_padded(int64_t R, int NL) {
     return (R + 4 * rs - 1) / (4 * rs) * (4 * rs);
 }
 
-int launch_fused_sampler(const __half* a16, int64_t R, int Kc, const __half* w16, int NL, float inv_t, uint64_t seed,
-                         uint64_t offset, int64_t* out, cudaStream_t st) {
+int64_t fused_sampler_mask_scratch_bytes(int64_t R, int NL) {
+    // the slot count (256 bytes) + one int per slot: a slot covers 4 rows of the padded feature buffer
+    return 256 + (fused_sampler_rows_padded(R, NL) + 255) / 256 * 256;
+}
+
+static int launch_fused_sampler_impl(const __half* a16, int64_t R, int Kc, const __half* w16, int NL, float inv_t,
+                                     uint64_t seed, uint64_t offset, const uint8_t* mask, void* mask_scratch, int64_t* out,
+                                     cudaStream_t st) {
     PB_CHECK(Kc % 8 == 0 && Kc <= 64 * SMP_MAX_KB, "fused sampler: c_out=%d unsupported (<= %d, multiple of 8)", Kc, 64 * SMP_MAX_KB);
     PB_CHECK(R * (int64_t)NL < (1ll << 31), "fused sampler: rows*labels >= 2^31 would split the torch kernel (unsupported)");
     PB_CHECK(offset % 4 == 0, "philox offset must be a multiple of 4");
@@ -384,34 +474,65 @@ int launch_fused_sampler(const __half* a16, int64_t R, int Kc, const __half* w16
             const int rs = (int)(rng.stride / NL);
             const int n_blocks = (int)((R + 4 * (int64_t)rs - 1) / (4 * (int64_t)rs));
             const int tpb = (rs + SH_JJ - 1) / SH_JJ;
+            int* count = nullptr;
+            int* slots = nullptr;
+            if (mask) {
+                count = reinterpret_cast<int*>(mask_scratch);
+                slots = reinterpret_cast<int*>(reinterpret_cast<uint8_t*>(mask_scratch) + 256);
+                const int n_slots = n_blocks * rs;
+                PB_CUDA(cudaMemsetAsync(count, 0, sizeof(int), st));
+                masked_slot_list_kernel<<<ceil_div(n_slots, 256), 256, 0, st>>>(mask, R, rs, n_slots, slots, count);
+                PB_LAUNCH_CHECK();
+            }
             static DeviceOnce attr2;
             if (attr2.first()) {
-                PB_CUDA(cudaFuncSetAttribute(fused_sampler_shared_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SH_SMEM));
+                PB_CUDA(cudaFuncSetAttribute(fused_sampler_shared_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SH_SMEM));
+                PB_CUDA(cudaFuncSetAttribute(fused_sampler_shared_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SH_SMEM));
     }
             ProfScope prof("fused_sampler", 2.0 * (double)R * (double)NL * (double)Kc, st);
             CUtensorMap tf, tw;
             const int64_t dims[4] = {Kc, 4, rs, n_blocks};
             const int64_t strides[3] = {(int64_t)rs * Kc * 2, (int64_t)Kc * 2, 4 * (int64_t)rs * Kc * 2};
-            const int box[4] = {64, 4, SH_JJ, 1};
+            const int box[4] = {64, 4, mask ? 1 : SH_JJ, 1};
             PB_TRY(make_tmap_f16_nd(&tf, a16, 4, dims, strides, box));
             PB_TRY(make_tmap_f16_2d(&tw, w16, NL, Kc, Kc, 128));
-            fused_sampler_shared_kernel<<<n_blocks * tpb, SH_THREADS, SH_SMEM, st>>>(tf, tw, (int)R, NL, Kc, rs, tpb, inv_t, rng, out);
+            if (mask)
+                fused_sampler_shared_kernel<true><<<n_blocks * tpb, SH_THREADS, SH_SMEM, st>>>(tf, tw, (int)R, NL, Kc, rs, tpb, inv_t, rng,
+                                                                                             slots, count, mask, out);
+            else
+                fused_sampler_shared_kernel<false><<<n_blocks * tpb, SH_THREADS, SH_SMEM, st>>>(tf, tw, (int)R, NL, Kc, rs, tpb, inv_t, rng,
+                                                                                              nullptr, nullptr, nullptr, out);
             PB_LAUNCH_CHECK();
             return 0;
         }
     }
     static DeviceOnce attr_set;
     if (attr_set.first()) {
-        PB_CUDA(cudaFuncSetAttribute(fused_sampler_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMP_SMEM));
+        PB_CUDA(cudaFuncSetAttribute(fused_sampler_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMP_SMEM));
+        PB_CUDA(cudaFuncSetAttribute(fused_sampler_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMP_SMEM));
     }
     ProfScope prof("fused_sampler", 2.0 * (double)R * (double)NL * (double)Kc, st);
     CUtensorMap ta, tw;
     PB_TRY(make_tmap_f16_2d(&ta, a16, R, Kc, Kc, 128));
     PB_TRY(make_tmap_f16_2d(&tw, w16, NL, Kc, Kc, SMP_BN));
     TorchPhilox rng = make_torch_philox(seed, offset, R * (int64_t)NL);
-    fused_sampler_kernel<<<ceil_div(R, 128), SMP_THREADS, SMP_SMEM, st>>>(ta, tw, (int)R, NL, Kc, inv_t, rng, out);
+    if (mask)
+        fused_sampler_kernel<true><<<ceil_div(R, 128), SMP_THREADS, SMP_SMEM, st>>>(ta, tw, (int)R, NL, Kc, inv_t, rng, mask, out);
+    else
+        fused_sampler_kernel<false><<<ceil_div(R, 128), SMP_THREADS, SMP_SMEM, st>>>(ta, tw, (int)R, NL, Kc, inv_t, rng, nullptr, out);
     PB_LAUNCH_CHECK();
     return 0;
+}
+
+int launch_fused_sampler(const __half* a16, int64_t R, int Kc, const __half* w16, int NL, float inv_t, uint64_t seed,
+                         uint64_t offset, int64_t* out, cudaStream_t st) {
+    return launch_fused_sampler_impl(a16, R, Kc, w16, NL, inv_t, seed, offset, nullptr, nullptr, out, st);
+}
+
+int launch_fused_sampler_masked(const __half* a16, int64_t R, int Kc, const __half* w16, int NL, float inv_t, uint64_t seed,
+                                uint64_t offset, const uint8_t* mask, void* mask_scratch, int64_t* tokens_inout, cudaStream_t st) {
+    PB_CHECK(mask != nullptr && mask_scratch != nullptr, "masked sampler: mask and scratch are required");
+    return launch_fused_sampler_impl(a16, R, Kc, w16, NL, inv_t, seed, offset, mask, mask_scratch, tokens_inout, st);
 }
 
 }  // namespace pb

@@ -108,10 +108,13 @@ __global__ void __launch_bounds__(192) vq_in_block_rw_kernel(const float* __rest
 // out_block: Conv2d(c0 -> 12, k=1) + PixelShuffle(2).  x NHWC fp32 [B,h2,w2,c0] -> img NCHW [B,3,2h2,2w2]; warp per position.
 // MODE (include/paella_b200.h PB200_IMG_*): 0 raw fp32 NCHW, 1 clamp(0,1) fp32 NCHW, 2 uint8 NHWC [B,2h2,2w2,3] with
 // save_image's rounding -- the callers' clamp / byte conversion passes fused into the store.
-template <int MODE>
+// COMPOSITE (pb200_vqgan_decode_composite): where pmask [B,2h2,2w2] is 0 the pixel is orig (fp32 NCHW, same size) instead of
+// the decoded value, put through the same MODE conversion.
+template <int MODE, bool COMPOSITE = false>
 __global__ void __launch_bounds__(256) vq_out_block_kernel(const float* __restrict__ x, const float* __restrict__ w,
                                                            const float* __restrict__ bias, int B, int h2, int w2, int c0,
-                                                           void* __restrict__ img_out) {
+                                                           void* __restrict__ img_out, const float* __restrict__ orig = nullptr,
+                                                           const uint8_t* __restrict__ pmask = nullptr) {
     const int lane = threadIdx.x & 31;
     const int64_t pos = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
     if (pos >= (int64_t)B * h2 * w2) return;
@@ -134,6 +137,10 @@ __global__ void __launch_bounds__(256) vq_out_block_kernel(const float* __restri
         const int y = rem / w2, xx = rem - y * w2;
         const int c = lane >> 2, d = lane & 3;
         v += bias[lane];
+        if constexpr (COMPOSITE) {
+            const int64_t px = ((int64_t)b * (2 * h2) + 2 * y + (d >> 1)) * (2 * w2) + 2 * xx + (d & 1);
+            if (pmask[px] == 0) v = orig[(((int64_t)b * 3 + c) * (2 * h2) + 2 * y + (d >> 1)) * (2 * w2) + 2 * xx + (d & 1)];
+        }
         if (MODE != 0) v = fminf(fmaxf(v, 0.f), 1.f);
         if (MODE == 2) {
             uint8_t* img = reinterpret_cast<uint8_t*>(img_out);
@@ -150,10 +157,11 @@ __global__ void __launch_bounds__(256) vq_out_block_kernel(const float* __restri
 // lane and position (ncu: LSU 63 %, 0.96 TB/s).  Here a thread owns a position: it pulls its row in 128-byte pieces (eight 16-byte
 // loads, consumed at once) and multiplies against the 12 x c0 weights staged in shared memory as [c/4][12] float4 (warp-wide
 // broadcast reads) -- 1.5 global loads + 18 shared loads per 72 FFMA.  Summation order: channels ascending per output.
-template <int MODE>
+template <int MODE, bool COMPOSITE = false>
 __global__ void __launch_bounds__(128) vq_out_block_tp_kernel(const float* __restrict__ x, const float* __restrict__ w,
                                                               const float* __restrict__ bias, int B, int h2, int w2, int c0,
-                                                              void* __restrict__ img_out) {
+                                                              void* __restrict__ img_out, const float* __restrict__ orig = nullptr,
+                                                              const uint8_t* __restrict__ pmask = nullptr) {
     extern __shared__ float4 w_s[];                      // [c0/4][12]: the 4 channel weights of output o
     const int nj = c0 >> 2;
     for (int i = threadIdx.x; i < nj * 12; i += blockDim.x) {
@@ -187,6 +195,10 @@ __global__ void __launch_bounds__(128) vq_out_block_tp_kernel(const float* __res
     for (int o = 0; o < 12; ++o) {
         float v = acc[o];
         const int c = o >> 2, d = o & 3;
+        if constexpr (COMPOSITE) {
+            const int64_t px = ((int64_t)b * (2 * h2) + 2 * y + (d >> 1)) * (2 * w2) + 2 * xx + (d & 1);
+            if (pmask[px] == 0) v = orig[(((int64_t)b * 3 + c) * (2 * h2) + 2 * y + (d >> 1)) * (2 * w2) + 2 * xx + (d & 1)];
+        }
         if (MODE != 0) v = fminf(fmaxf(v, 0.f), 1.f);
         if (MODE == 2) {
             uint8_t* img = reinterpret_cast<uint8_t*>(img_out);
@@ -660,8 +672,10 @@ int pb200_vqgan_decode(pb200_vqgan* m, const int64_t* indices, const float* late
     return pb200_vqgan_decode_ex(m, indices, latents_nchw, batch, h, w, img, PB200_IMG_F32_NCHW, workspace, workspace_bytes, stream);
 }
 
-int pb200_vqgan_decode_ex(pb200_vqgan* m, const int64_t* indices, const float* latents_nchw, int batch, int h, int w, void* img,
-                          int img_mode, void* workspace, int64_t workspace_bytes, void* stream) {
+// orig / pmask non-null: the last kernel composites (pb200_vqgan_decode_composite)
+static int vq_decode_impl(pb200_vqgan* m, const int64_t* indices, const float* latents_nchw, int batch, int h, int w, void* img,
+                          int img_mode, const float* orig, const uint8_t* pmask, void* workspace, int64_t workspace_bytes,
+                          void* stream) {
     PB_CHECK(m->blob != nullptr, "decode: weights not bound");
     PB_CHECK(img_mode >= 0 && img_mode <= 2, "decode: unknown image mode %d", img_mode);
     if (m->host_params_stale) PB_TRY(pb200_vqgan_sync_params(m, stream));
@@ -717,7 +731,17 @@ int pb200_vqgan_decode_ex(pb200_vqgan* m, const int64_t* indices, const float* l
     {
         ProfScope prof("vq_out_block", (double)M0 * (c0 * 4.0 + 48.0), st);
         const float *ow = m->w<float>(m->out_w), *ob = m->w<float>(m->out_b);
-        if (c0 % 32 == 0 && c0 <= 768) {         // thread per position, weights in shared memory
+        if (pmask) {
+            if (c0 % 32 == 0 && c0 <= 768) {
+                const size_t sm = (size_t)c0 * 48;
+                const unsigned g = (unsigned)ceil_div(M0, 128);
+                if (img_mode == PB200_IMG_U8_NHWC) vq_out_block_tp_kernel<2, true><<<g, 128, sm, st>>>(ws.xa, ow, ob, B, h0, w0, c0, img, orig, pmask);
+                else if (img_mode == PB200_IMG_F32_NCHW_CLAMP01) vq_out_block_tp_kernel<1, true><<<g, 128, sm, st>>>(ws.xa, ow, ob, B, h0, w0, c0, img, orig, pmask);
+                else vq_out_block_tp_kernel<0, true><<<g, 128, sm, st>>>(ws.xa, ow, ob, B, h0, w0, c0, img, orig, pmask);
+            } else if (img_mode == PB200_IMG_U8_NHWC) vq_out_block_kernel<2, true><<<ceil_div(M0, 8), 256, 0, st>>>(ws.xa, ow, ob, B, h0, w0, c0, img, orig, pmask);
+            else if (img_mode == PB200_IMG_F32_NCHW_CLAMP01) vq_out_block_kernel<1, true><<<ceil_div(M0, 8), 256, 0, st>>>(ws.xa, ow, ob, B, h0, w0, c0, img, orig, pmask);
+            else vq_out_block_kernel<0, true><<<ceil_div(M0, 8), 256, 0, st>>>(ws.xa, ow, ob, B, h0, w0, c0, img, orig, pmask);
+        } else if (c0 % 32 == 0 && c0 <= 768) {         // thread per position, weights in shared memory
             const size_t sm = (size_t)c0 * 48;
             const unsigned g = (unsigned)ceil_div(M0, 128);
             if (img_mode == PB200_IMG_U8_NHWC) vq_out_block_tp_kernel<2><<<g, 128, sm, st>>>(ws.xa, ow, ob, B, h0, w0, c0, img);
@@ -729,6 +753,19 @@ int pb200_vqgan_decode_ex(pb200_vqgan* m, const int64_t* indices, const float* l
         PB_LAUNCH_CHECK();
     }
     return 0;
+}
+
+int pb200_vqgan_decode_ex(pb200_vqgan* m, const int64_t* indices, const float* latents_nchw, int batch, int h, int w, void* img,
+                          int img_mode, void* workspace, int64_t workspace_bytes, void* stream) {
+    return vq_decode_impl(m, indices, latents_nchw, batch, h, w, img, img_mode, nullptr, nullptr, workspace, workspace_bytes, stream);
+}
+
+int pb200_vqgan_decode_composite(pb200_vqgan* m, const int64_t* indices, int batch, int h, int w, const float* orig_img,
+                                 const uint8_t* pixel_mask, void* img, int img_mode, void* workspace, int64_t workspace_bytes,
+                                 void* stream) {
+    PB_CHECK(indices != nullptr && orig_img != nullptr && pixel_mask != nullptr,
+             "decode_composite: indices, orig_img and pixel_mask are required");
+    return vq_decode_impl(m, indices, nullptr, batch, h, w, img, img_mode, orig_img, pixel_mask, workspace, workspace_bytes, stream);
 }
 
 }  // extern "C"

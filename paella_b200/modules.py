@@ -664,6 +664,37 @@ class Paella(nn.Module):
                                                    ptr(flat[lo:hi]), ptr(ws), ws.numel(), current_stream()), "pb200_paella_sample_tokens")
         return out
 
+    def sample_tokens_masked(self, feats: torch.Tensor, batch: int, h: int, w: int, cfg: Optional[float], temperature: float,
+                             known: torch.Tensor, mask: torch.Tensor, generator=None) -> torch.Tensor:
+        """``where(mask, sample_tokens(...), known)`` without drawing the kept rows: ``known`` int64 [B,H,W], ``mask``
+        bool/uint8 [B,H,W] (1 = regenerate).  The draw at a masked position is bit-identical to ``sample_tokens``'s and the
+        generator advances by the same amount, so a mask of all ones reproduces the unmasked sampler."""
+        self._ensure_packed()
+        L = lib()
+        dev = self._device()
+        with torch.cuda.device(dev):
+            out = known.to(device=dev, dtype=torch.int64).reshape(batch, h, w).clone()
+            m8 = mask.to(device=dev).reshape(batch, h, w)
+            m8 = (m8 if m8.dtype == torch.bool else m8 != 0).contiguous().view(torch.uint8)      # bool storage is 0 / 1 bytes
+            ws = self._ws(L.pb200_paella_workspace_bytes(self._handle, batch, h, w, 1))
+            n = batch * h * w
+            chunks = ops.philox_row_chunks(n, self.num_labels)       # the same pieces, offsets and draws as sample_tokens
+            ops.skip_philox_for_split(chunks, n * self.num_labels, dev, generator)
+            flat, mflat = out.view(-1), m8.view(-1)
+            for lo, hi in chunks:
+                seed, off = ops.take_philox((hi - lo) * self.num_labels, dev, generator)
+                if len(chunks) == 1:
+                    f = feats
+                elif cfg is not None:
+                    f = torch.cat([feats[lo:hi], feats[n + lo:n + hi]])
+                else:
+                    f = feats[lo:hi]
+                check(L.pb200_paella_sample_tokens_masked(self._handle, ptr(f), 1, hi - lo, 1 if cfg is not None else 0,
+                                                          float(cfg) if cfg is not None else 0.0, float(temperature), seed, off,
+                                                          ptr(mflat[lo:hi]), ptr(flat[lo:hi]), ptr(ws), ws.numel(),
+                                                          current_stream()), "pb200_paella_sample_tokens_masked")
+        return out
+
     def forward(self, x, r, byt5, clip=None, clip_image=None, x_cat=None, **kwargs):
         """ref/src/modules.py:263-275 / ref/utils/modules.py:268-282: logits [B, num_labels, H, W] fp32."""
         if x_cat is not None:

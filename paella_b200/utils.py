@@ -3,6 +3,7 @@
   sample()               ref/src/utils.py:35-55
   sample_distributed()   ref/src_distributed/utils.py:97-126   (init_x, per-step cfg, sampling_conditional_steps)
   sample_notebook()      paella_inference.ipynb cell 3          (mode, attn_weights, returns intermediates)
+  sample_masked()        sample_notebook() regenerating only where a mask is set (inpainting / outpainting)
 
 Per step the reference runs two forwards, materialises 2 x [B,8192,H,W] fp32 logits and makes ~20 passes
 over them.  Here: conditional and unconditional rows run as ONE batch of 2B through the denoiser (their
@@ -18,6 +19,7 @@ from typing import Dict, Optional, Sequence, Tuple
 import torch
 
 from . import ops
+from ._lib import PaellaB200Error
 from .modules import Paella
 
 
@@ -27,13 +29,21 @@ def _zeros_like_inputs(inputs: Dict[str, torch.Tensor]):
 
 def _sample_core(model: Paella, model_inputs, latent_shape, unconditional_inputs, init_x, steps, renoise_steps, temperature,
                  cfgs, t_start, t_end, sampling_conditional_steps, mode, attn_weights, exact, collect, sampling_quant_steps=None,
-                 codebook=None):
+                 codebook=None, known=None, mask=None):
+    """``known`` int64 [B,H,W] / ``mask`` bool [B,H,W] on the model's device (1 = regenerate), or both None: masked
+    sampling keeps ``known`` wherever the mask is 0, in the start state and after every draw; the renoise is unchanged
+    because the noise it draws from equals ``known`` there."""
     B, H, W = latent_shape
     dev = model._device()
     use_cfg_any = cfgs is not None
     with torch.inference_mode():
         init_noise = ops.randint(model.num_labels, (B, H, W), dev)
-        sampled = init_x.to(dev) if init_x is not None else init_noise.clone()
+        if mask is not None:
+            init_noise = torch.where(mask, init_noise, known)
+        if init_x is not None:
+            sampled = torch.where(mask, init_x.to(dev), known) if mask is not None else init_x.to(dev)
+        else:
+            sampled = init_noise.clone()
         t_list = torch.linspace(t_start, t_end, steps + 1)
         temperatures = torch.linspace(temperature[0], temperature[1], steps)
         groups = [model_inputs] + ([unconditional_inputs] if use_cfg_any else [])
@@ -56,7 +66,9 @@ def _sample_core(model: Paella, model_inputs, latent_shape, unconditional_inputs
             r = torch.full((tokens.shape[0],), t, dtype=torch.float32, device=dev)
             feats = model.features(tokens, r, cond, attn_weights, B if attn_weights is not None else 0, cfg_pairs=guided)
             cfg_i = float(cfgs[i]) if guided else None
-            if mode == "multinomial" and not exact:
+            if mode == "multinomial" and not exact and mask is not None:
+                sampled = model.sample_tokens_masked(feats, B, H, W, cfg_i, float(temperatures[i]), known, mask)
+            elif mode == "multinomial" and not exact:
                 sampled = model.sample_tokens(feats, B, H, W, cfg_i, float(temperatures[i]))
             else:
                 n = B * H * W
@@ -68,6 +80,8 @@ def _sample_core(model: Paella, model_inputs, latent_shape, unconditional_inputs
                     sampled = ops.resample_quant(lc, lu, cfg_i if guided else 0.0, float(temperatures[i]), codebook)
                 else:
                     sampled = ops.resample_logits(lc, lu, cfg_i if guided else 0.0, float(temperatures[i]), mode)
+                if mask is not None:
+                    sampled = torch.where(mask, sampled, known)
             if collect:
                 intermediates.append(sampled)
             if i < renoise_steps:
@@ -154,3 +168,41 @@ def sample_notebook(model, model_inputs, latent_shape, unconditional_inputs=None
     return _sample_core(model, model_inputs, tuple(latent_shape), unconditional_inputs, init_x, steps, renoise_steps,
                         temperature, cfgs, t_start, t_end, sampling_conditional_steps, mode, attn_weights, exact, True,
                         sampling_quant_steps, codebook)
+
+
+def _masked_inputs(model, known, mask):
+    """Validate (known [B,H,W] tokens, mask [B,H,W] or [H,W]) and move them to the model's device: int64 and bool [B,H,W]."""
+    if known.dim() != 3:
+        raise PaellaB200Error(f"sample_masked: known must be [B,H,W] tokens, got shape {tuple(known.shape)}")
+    B, H, W = known.shape
+    if tuple(mask.shape) not in ((B, H, W), (H, W)):
+        raise PaellaB200Error(f"sample_masked: mask has shape {tuple(mask.shape)}, expected {(B, H, W)} or {(H, W)}")
+    dev = model._device()
+    known = known.to(device=dev, dtype=torch.int64).contiguous()
+    mask = mask.to(device=dev).bool().expand(B, H, W).contiguous()
+    return known, mask
+
+
+def sample_masked(model, model_inputs, known, mask, unconditional_inputs=None, init_x=None, steps=12, renoise_steps=None,
+                  temperature=(0.7, 0.3), cfg=(8.0, 8.0), mode='multinomial', t_start=1.0, t_end=0.0,
+                  sampling_conditional_steps=None, sampling_quant_steps=None, attn_weights=None, exact=False, vqmodel=None):
+    """Inpainting / outpainting on token grids: ``sample_notebook`` over the latent shape of ``known`` (int64 [B,H,W])
+    that regenerates only the positions where ``mask`` ([B,H,W] or [H,W], broadcast over the batch) is 1 -- the meaning
+    of ``mask`` in ``Paella.add_noise`` (ref/src/modules.py:277-283).  Returns (tokens, intermediates) like
+    ``sample_notebook``; kept positions hold ``known`` in the result and in every intermediate.
+
+    The torch generator is consumed exactly as by the unmasked loop of the same shape (every draw is full-size), so a
+    mask of all ones reproduces ``sample_notebook`` from the same seed.  On the fused path the sampler spends work only on
+    the positions to regenerate; ``exact=True``, ``mode='argmax'`` and ``'quant'`` merge after the draw."""
+    known, mask = _masked_inputs(model, known, mask)
+    if sampling_conditional_steps is None:
+        sampling_conditional_steps = steps
+    if renoise_steps is None:
+        renoise_steps = steps - 1
+    if unconditional_inputs is None:
+        unconditional_inputs = _zeros_like_inputs(model_inputs)
+    cfgs = torch.linspace(cfg[0], cfg[1], steps).tolist() if cfg is not None else None
+    codebook = vqmodel.vquantizer.codebook.weight.data if vqmodel is not None else None
+    return _sample_core(model, model_inputs, tuple(known.shape), unconditional_inputs, init_x, steps, renoise_steps,
+                        temperature, cfgs, t_start, t_end, sampling_conditional_steps, mode, attn_weights, exact, True,
+                        sampling_quant_steps, codebook, known, mask)

@@ -279,6 +279,34 @@ class VQModel(nn.Module):
         (``mul(255).add_(0.5).clamp_(0,255).to(uint8)`` on the HWC view), fused into the decoder's last kernel."""
         return self._decode(x, None, _lib.IMG_U8_NHWC)
 
+    def decode_composite(self, x, orig, pixel_mask, output="uint8"):
+        """Decode indices x [B,h,w] and paste the original image back: pixels where ``pixel_mask`` ([B,4h,4w] or [4h,4w],
+        1 = decoded) is 0 come from ``orig`` (fp32 NCHW [B,3,4h,4w]) through the same conversion as the decoded ones.
+        ``output``: 'uint8' (NHWC, as ``decode_indices_u8``), 'clamp' or 'raw' (fp32 NCHW).  One fused last kernel."""
+        mode = {"uint8": _lib.IMG_U8_NHWC, "clamp": _lib.IMG_F32_NCHW_CLAMP01, "raw": _lib.IMG_F32_NCHW}.get(output)
+        if mode is None:
+            raise ValueError(f"output={output!r}: expected 'uint8', 'clamp' or 'raw'")
+        self._ensure_packed()
+        L, dev = lib(), self._device()
+        with torch.cuda.device(dev):
+            idx = x.to(device=dev, dtype=torch.int64).contiguous()
+            B, h, w = idx.shape
+            if tuple(orig.shape) != (B, 3, 4 * h, 4 * w):
+                raise PaellaB200Error(f"decode_composite: orig has shape {tuple(orig.shape)}, expected {(B, 3, 4 * h, 4 * w)}")
+            if tuple(pixel_mask.shape) not in ((B, 4 * h, 4 * w), (4 * h, 4 * w)):
+                raise PaellaB200Error(f"decode_composite: pixel_mask has shape {tuple(pixel_mask.shape)}, expected "
+                                      f"{(B, 4 * h, 4 * w)} or {(4 * h, 4 * w)}")
+            orig = orig.to(device=dev, dtype=torch.float32).contiguous()
+            pm = pixel_mask.to(device=dev).bool().expand(B, 4 * h, 4 * w).to(torch.uint8).contiguous()
+            if mode == _lib.IMG_U8_NHWC:
+                img = torch.empty(B, 4 * h, 4 * w, 3, dtype=torch.uint8, device=dev)
+            else:
+                img = torch.empty(B, 3, 4 * h, 4 * w, dtype=torch.float32, device=dev)
+            ws = self._ws(L.pb200_vqgan_workspace_bytes(self._handle, B, 4 * h, 4 * w))
+            check(L.pb200_vqgan_decode_composite(self._handle, ptr(idx), B, h, w, ptr(orig), ptr(pm), ptr(img), mode, ptr(ws),
+                                                 ws.numel(), current_stream()), "pb200_vqgan_decode_composite")
+        return img
+
     def forward(self, x, quantize=False):
         qe, x, _, vq_loss = self.encode(x, quantize)
         return self.decode(qe), vq_loss
